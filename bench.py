@@ -23,6 +23,11 @@ Numbers in the JSON line (all: max over ranks, throughput = workers x K / max el
              with `--strict_steps` (the next pull waits for the acknowledgement of the previous push).
   roofline : achieved fraction of the NVLink / HBM / tensor-core rooflines from MEASURED_PEAKS.json.
 
+--dump-outputs DIR: after the device-timed region, the chief worker writes what its last step returned (`loss.npy`,
+`correct.npy`) and the variables on the ps shards (`var_<name>.npy`, "/" in a name becomes "__") as float32. Data and
+initial variables are seeded, so two builds run with the same arguments start from identical inputs; with more than
+one step in flight (`--lanes`) the staleness of each pull depends on timing, so compare with a tolerance.
+
 Steps in flight: a worker keeps `--lanes` (default 12, the CLI's default too) steps in flight on its GPU — bounded-
 staleness asynchronous SGD: every step still pulls, computes, pushes and is applied on the ps individually.
 """
@@ -43,6 +48,7 @@ REFERENCE_UNAVAILABLE = (
     "`pip install --target baseline/_ref /root/reference` fails with 'not installable'"
 )
 NVLINK_GBS = 770.0   # measured peer-copy bandwidth per direction per GPU (profiling recipe)
+DUMP_MAX_BYTES = 60 << 20   # --dump-outputs: array data in all (the .npy headers stay well inside 64 MB)
 
 
 def parse_args(argv=None):
@@ -71,6 +77,9 @@ def parse_args(argv=None):
     p.add_argument("--ps_row_blocks", type=int, default=4)
     p.add_argument("--skip_e2e", action="store_true")
     p.add_argument("--skip_parity", action="store_true")
+    p.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                   help="after the device-timed steps, write the result of their last step and the variables it left "
+                        "on the ps as DIR/<name>.npy (float32), to compare two builds output for output")
     return p.parse_args(argv)
 
 
@@ -220,8 +229,8 @@ def main(argv=None) -> int:
     phase = [0]
     sync_ms = []
 
-    def full_sync(restart: bool = True):
-        """barrier + torch.cuda.synchronize() on every rank.
+    def full_sync(restart: bool = True, at_rest=None):
+        """barrier + torch.cuda.synchronize() on every rank; `at_rest()` runs then, before any serve kernel restarts.
 
         A resident persistent PS kernel makes a device synchronise hang, and — because CUDA loads kernels lazily —
         even the *first launch* of any new kernel (an NCCL barrier, a torch op) in that context can deadlock
@@ -249,6 +258,8 @@ def main(argv=None) -> int:
                     print(f"[ps_stats] sync {ph} rank={rank} shard={ps.task_index} {json.dumps(st)}", file=sys.stderr, flush=True)
         barrier()
         torch.cuda.synchronize()
+        if at_rest is not None:
+            at_rest()
         if restart:
             for ps in ps_list:
                 ps.restart()
@@ -300,6 +311,27 @@ def main(argv=None) -> int:
         assert len(outs) == n, (len(outs), n)
         return dt
 
+    def dump_outputs():
+        """The result of the last device-timed step and the variables the timed steps left on the ps shards (read
+        while no serve kernel runs). Larger than DUMP_MAX_BYTES in all: a fixed, seeded sample of every array."""
+        if worker is None or not worker.is_chief:
+            return
+        import numpy as np
+        last = worker.last_resident_result()
+        arrays = {"loss": np.array([last.loss], np.float32), "correct": np.array([last.correct], np.float32)}
+        for name, t in worker.read_variables().items():
+            arrays["var_" + name.replace("/", "__")] = t.numpy().astype(np.float32)
+        total = sum(a.nbytes for a in arrays.values())
+        if total > DUMP_MAX_BYTES:
+            rng = np.random.default_rng(0)
+            for name, a in arrays.items():
+                n = int(a.size * DUMP_MAX_BYTES / total)
+                if n < a.size:
+                    arrays[name] = a.reshape(-1)[np.sort(rng.choice(a.size, max(n, 1), replace=False))]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+
     elapsed_ms = host_enqueue_ms = e2e_s = 0.0
     par = {"dev_ms": 0.0, "e2e_s": 0.0, "strict_ms": 0.0}
     h2d_bytes = d2h_bytes = 0
@@ -322,7 +354,7 @@ def main(argv=None) -> int:
         launches_before = worker.kernel_launches()
         elapsed_ms, host_enqueue_ms = device_timed(K)
         launches = worker.kernel_launches() - launches_before + (0 if engine == "fused" else 1)   # (+ wait_ack kernel)
-    full_sync()
+    full_sync(at_rest=dump_outputs if args.dump_outputs else None)
     if os.environ.get("DM_FUSED_DEBUG_TS") == "1" and worker is not None and getattr(worker, "_fx_dbg", None) is not None:
         from bench_tools.fused_phases import print_stamps   # in-kernel phase stamps of the timed launch (stderr)
         import contextlib

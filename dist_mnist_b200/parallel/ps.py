@@ -498,6 +498,23 @@ class ParameterServer:
                 self.serve_once()      # one-shot mode as a stand-alone task: apply whatever has arrived
             time.sleep(poll_s)
         self.stop()
+        if exit_when_done:
+            self._leave_rendezvous()
+
+    def _leave_rendezvous(self, timeout_s: float = 30.0) -> None:
+        """ps 0 hosts the rendezvous store, so it keeps it up until the other tasks have made their last call to it:
+        the other ps tasks leave their serve loops at about the same time and poll the store until then, and a worker
+        adds to `session/workers_done` only after its done word has reached the shards. Bounded: a task that died
+        never signs off."""
+        if not self.rdv.is_master:
+            self.rdv.add("session/ps_left", 1)
+            return
+        deadline = time.time() + timeout_s
+        while (self.rdv.add("session/ps_left", 0) < self.cluster.num_ps - 1
+               or self.rdv.add("session/workers_done", 0) + len(self._dead) < self.n_workers):
+            if time.time() > deadline:
+                break
+            time.sleep(0.01)
 
     def close(self) -> None:
         self.stop()

@@ -793,6 +793,20 @@ class Worker:
         N.check(self.lib.dm_exec_run_resident(self._exec, n_steps, x_base_ptr, y_base_ptr, x_row_bytes, y_row_bytes,
                                               n_rows, self.batch, start), "run resident")
 
+    def last_resident_result(self) -> StepOutput:
+        """Result of the final step of the most recent `run_resident` (waits for it)."""
+        if self.engine == "fused":
+            n = C.c_uint64()
+            N.check(self.lib.dm_fexec_resident_results(self._fexec, None, 2 ** 64 - 1, C.byref(n)), "resident results")
+            if n.value == 0:
+                raise N.NativeError("no resident run to report on")
+            res = (N.StepResult * n.value)()
+            N.check(self.lib.dm_fexec_resident_results(self._fexec, C.addressof(res), n.value, C.byref(n)),
+                    "resident results")
+            r = res[n.value - 1]
+            return StepOutput(r.loss, r.global_step, r.correct, r.seq)
+        return self.result(int(self.lib.dm_exec_submitted(self._exec)), wait=True)
+
     def last_elapsed_ms(self) -> float:
         """Fused engine: device time (CUDA events recorded natively right around the launch) of the most recent
         `run_resident(..., timed=True)`."""
